@@ -18,6 +18,9 @@ One "step" = one pass of the hot path over the whole record batch:
             gives the configs[1]-sized forest on CICIDS-shaped rows (a stress case: 1.5 M nodes, see DESIGN.md).
 `--scaling`: weak (rows per GPU fixed, default) | strong (the workload's global rows sharded over the ranks; every N prints
             `forest_hash`, equal for every N: integer histograms + global-row-keyed RNG).
+`--dump-outputs DIR`: after the timed steps, the last timed step's results (predictions, probabilities, raw votes, confusion,
+            macro-F1, thresholds and forest; the stream workload: predictions) as DIR/<name>.npy, float64, at most 64 MB in all
+            (a seeded sample of rows when larger).  The inputs are seeded, so equal arguments give equal inputs on every run.
 Launch: python bench.py --gpus N --steps K --warmup W   (N>1 under torchrun, one rank per GPU).
 """
 import argparse
@@ -69,6 +72,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sklearn", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64)")
     a = ap.parse_args()
     kind, rows, classes, trees, depth, bins, dtype, site = WORKLOADS[a.workload]
     a.kind, a.site = kind, site
@@ -147,6 +152,36 @@ def forest_hash(ex):
     internal = np.asarray(ex["is_leaf"]) == 0
     h.update(np.ascontiguousarray(np.asarray(ex["gain"], np.float64)[internal]).tobytes())
     return h.hexdigest()[:16]
+
+
+DUMP_BYTES = 60 << 20          # all --dump-outputs files together, .npy headers included, stay under 64 MB
+
+
+def forest_outputs(ex):
+    """the canonical forest export as float64-exact arrays: the uint64 left-set masks are split into their 32-bit words."""
+    return {"forest_" + k: (np.asarray(v, np.uint64).view(np.uint32) if k == "mask" else v) for k, v in ex.items()}
+
+
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: write each output of the last timed step as <out_dir>/<name>.npy in float64, so that two builds can be
+    compared array for array.  When the arrays exceed DUMP_BYTES, every array over 1 MB keeps the same fraction of its rows,
+    chosen by a generator seeded with its row count: arrays with one row per test record (prediction, probability,
+    rawPrediction) keep the same records, and two runs of the same arguments keep the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (v.detach().to(torch.float64).cpu().numpy() if torch.is_tensor(v) else np.asarray(v, np.float64))
+              for k, v in outputs.items()}
+    big = [k for k, v in arrays.items() if v.ndim and v.nbytes > (1 << 20)]
+    big_bytes = sum(arrays[k].nbytes for k in big)
+    room = DUMP_BYTES - sum(v.nbytes + 4096 for k, v in arrays.items() if k not in big) - 4096 * len(big)
+    if big_bytes > room:
+        rows = {}
+        for k in big:
+            n = arrays[k].shape[0]
+            if n not in rows:
+                rows[n] = np.sort(np.random.default_rng(n).choice(n, int(n * room / big_bytes), replace=False))
+            arrays[k] = arrays[k][rows[n]]
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
@@ -244,7 +279,9 @@ def run_reference_stream(a, wl, threads):
         cpu_stream_pass(wl, plan, fo, meta, rec_np)
     t = []
     for _ in range(a.steps):
-        t0 = time.perf_counter(); cpu_stream_pass(wl, plan, fo, meta, rec_np); t.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); pred = cpu_stream_pass(wl, plan, fo, meta, rec_np); t.append(time.perf_counter() - t0)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"prediction": pred})
     ms = 1e3 * sum(t) / len(t)
     v = a.cpu_rows / (ms / 1e3)
     line = {"impl": "reference", "metric": "flow-records/sec encode+predict (stream)", "value": v, "unit": "records/s", "n_gpus": a.gpus,
@@ -285,7 +322,9 @@ def run_reference(a):
         cpu_pass(wl, rec_np, dicts, a)
     t, f1, ph = [], 0.0, {}
     for _ in range(a.steps):
-        t0 = time.perf_counter(); f1, _, _ = cpu_pass(wl, rec_np, dicts, a, ph); t.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); f1, pred, ex = cpu_pass(wl, rec_np, dicts, a, ph); t.append(time.perf_counter() - t0)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"prediction": pred, "macro_f1": f1, **forest_outputs(ex)})
     ms = 1e3 * sum(t) / len(t)
     v = a.cpu_rows / (ms / 1e3)
     cfg = wl.describe(world, a.rows, a.rows * world if a.scaling == "weak" else a.rows)
@@ -383,7 +422,7 @@ def step_resident(wl, rec, dicts, a, grp, keep=None):
     cm = bdist.all_reduce_sum_(fr.confusion_matrix(pred, yte.to(torch.float64), C), grp)   # R10
     f1 = fr.metrics_from_confusion(cm.cpu().numpy())["macroF1"]
     if keep is not None:
-        keep.update(model=model, pred=pred)
+        keep.update(model=model, pred=pred, raw=raw, prob=prob, confusion=cm, macro_f1=f1)
     return f1, nte, model.train_stats, model.n_nodes
 
 
@@ -517,6 +556,13 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if a.dump_outputs:                                          # rank 0: its own test rows, and the global forest
+        model = keep["model"]
+        out = {"prediction": keep["pred"], "rawPrediction": keep["raw"], "probability": keep["prob"], "confusion": keep["confusion"],
+               "macro_f1": keep["macro_f1"], "thresholds": model.thresholds, **forest_outputs(model.export())}
+        if e2e is not None:
+            out["e2e_prediction"] = host_pred
+        dump_outputs(a.dump_outputs, out)
 
     # ---- roofline of the dominant kernel (CUDA events on the launching stream, inside the timed steps) -----
     peaks = {}
@@ -684,6 +730,8 @@ def run_stream(a, wl, dev, grp, world, rank, local):
         if world > 1:
             dist.destroy_process_group()
         return
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"prediction": pred})
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
              "dtype", "data", "config"}
@@ -42,6 +45,44 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                          capture_output=True, text=True, timeout=300, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def _dump(tmp_path, tag, *args):
+    out = tmp_path / tag
+    run = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(out)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert run.returncode == 0, run.stderr[-2000:]
+    files = sorted(os.listdir(out))
+    assert sum(os.path.getsize(out / f) for f in files) <= 64 << 20
+    arrays = {f[:-4]: np.load(out / f) for f in files}
+    assert all(v.dtype in (np.float32, np.float64) for v in arrays.values())
+    return arrays
+
+
+def _assert_same(a, b):
+    assert sorted(a) == sorted(b)
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+
+
+def test_reference_arm_dumps_the_same_outputs_whatever_the_step_count(tmp_path):
+    args = ["--impl", "reference", "--cpu-rows", "4000", "--trees", "4", "--depth", "4"]
+    a = _dump(tmp_path, "a", *args, "--steps", "1", "--warmup", "0")
+    b = _dump(tmp_path, "b", *args, "--steps", "2", "--warmup", "1")
+    _assert_same(a, b)
+    assert {"prediction", "macro_f1", "forest_nid", "forest_counts", "forest_mask"} <= set(a) and len(a["prediction"]) > 900
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_same_outputs_whatever_the_step_count(tmp_path):
+    args = ["--rows", "30000", "--trees", "4", "--depth", "6", "--no-cpu-baseline"]
+    a = _dump(tmp_path, "a", *args, "--steps", "1", "--warmup", "0")
+    b = _dump(tmp_path, "b", *args, "--steps", "3", "--warmup", "2")
+    _assert_same(a, b)
+    assert np.array_equal(a["prediction"], a["e2e_prediction"]) and len(a["prediction"]) > 6000
+    C = a["confusion"].shape[0]                                 # confusion[label, prediction] over the same test rows
+    assert a["probability"].shape == a["rawPrediction"].shape == (len(a["prediction"]), C)
+    assert np.array_equal(a["confusion"].sum(0), np.bincount(a["prediction"].astype(np.int64), minlength=C))
 
 
 def test_gpu_arm_keys_are_emitted_by_bench_source():
